@@ -1,16 +1,19 @@
 #!/usr/bin/env python
 """bench.py — Neural-Object-Field train-step throughput (BASELINE.json metric: NeRF train rays/s, steps/s, % HBM roofline).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config C2|C1|C3|C5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config C2|C1|C3|C5] [--dump-outputs DIR]
 
 Workload (config.workload): BASELINE.json configs[1] "C2" — milk-jug-shaped synthetic sequence, 200 frames 640x480,
 2048 rays x 128 samples (64 occupied-voxel + 64 around-depth), hash grid L=16 T=2^19 finest 256, MLP = the reference
 NeRFSmall (SDF 2x64, colour 3x64), AMP on, pose refinement on. A step = one NerfRunner.train_loop (gather batch from the
 ray pool -> pose correction -> ray march -> fused forward/loss/backward -> pose backward -> Adam).
-  value : rays/s with the ray pool resident in HBM: blocks of K steps (NerfRunner.train_steps: one CUDA graph per 10 steps, batch
-          cursor on the device) x R repetitions, each block CUDA-event timed between barrier + synchronize; median of the max over ranks.
-  e2e   : same metric through the public API from HOST buffers: every step copies its batch from pinned host memory
-          (what the reference does after add_new_frames, nerf_runner.py:431: rays live on the CPU) and reads the loss back.
+  value : rays/s with the ray pool resident in HBM: K = --steps timed steps (NerfRunner.train_steps: one CUDA graph per 10 steps,
+          batch cursor on the device), CUDA-event timed between barrier + synchronize; the max over ranks.
+  e2e   : same metric through the public API from HOST buffers, K more timed steps: every step copies its batch from pinned host
+          memory (what the reference does after add_new_frames, nerf_runner.py:431: rays live on the CPU) and reads the loss back.
+  --dump-outputs DIR : after the K timed steps of `value`, what a caller of train_steps has from the last of them, as DIR/<name>.npy
+          (float32): the step's loss terms and the trained parameters, the hash table as a fixed seeded sample of its rows. The
+          workload and the number of steps before the dump depend on the arguments only, so two builds can be compared output for output.
   roofline : the fused step kernel alone, algorithmic bytes P*64*L*C + N*60 (SURVEY.md 8d) / its mean launch time (`achieved`, `frac`);
           the whole step incl. the 34 B/param Adam stream (`achieved_step`, `frac_step`); `traffic` = ncu dram bytes of this config.
   cpu_baseline : the oracle port (oracle/nof_oracle.py, torch fp32 on all host cores) at the workload's full batch (fewer steps).
@@ -71,10 +74,9 @@ def optimizer_bytes(n_params):
 
 class ClockSampler(threading.Thread):
     """SM clock and throttle reasons sampled DURING the timed region (B200_PROFILING.md clocks line) through NVML (the library
-    behind nvidia-smi) every 25 ms — the timed region is REPS blocks of K steps and lasts >= ~0.4 s, so it still gets a dozen or
-    more samples, while a query (50 us .. 2 ms of host time) can no longer land in every block (round 1 polled every 2 ms inside a
-    6 ms region and halved the 8-GPU headline). Falls back to spawning `nvidia-smi --query-gpu=clocks.sm,...` when pynvml is not
-    importable."""
+    behind nvidia-smi) every 25 ms — rarely enough that a query (50 us .. 2 ms of host time) does not land in every step (polling
+    every 2 ms inside a 6 ms region once halved the 8-GPU headline); a region shorter than 25 ms gets one sample. Falls back to
+    spawning `nvidia-smi --query-gpu=clocks.sm,...` when pynvml is not importable."""
 
     REASONS = ((0x8, 'hw_slowdown'), (0x40, 'hw_thermal_slowdown'), (0x20, 'sw_thermal_slowdown'), (0x4, 'sw_power_cap'))
 
@@ -324,28 +326,25 @@ def measure_config(args, c, name, rank, world, local_rank, dev, with_kernel=True
     N, K = c['N'], args.steps
     n_params = sum(int(sg['param'].numel()) for sg in runner.adam_segs.values())
 
-    # ---- warm-up: >= W steps, then on to a step index = 1 (mod 10) so that a timed K-step block is K/10 whole graph replays
+    def align():                                            # on to a step index = 1 (mod 10): K timed steps are whole graph replays
+        while runner.global_step % 10 != 1:
+            runner.train_steps(1)
+
+    # ---- warm-up: >= W steps, then the same K steps as the timed region once, which captures its graphs outside of it
     runner.train_steps(max(args.warmup, 3))
-    while runner.global_step % 10 != 1:
-        runner.train_steps(1)
-    runner.train_steps(K)                                   # captures the block graphs outside the timed region
-    torch.cuda.synchronize()
-    ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    ev0.record(); runner.train_steps(K); ev1.record(); torch.cuda.synchronize()
-    est = max(ev0.elapsed_time(ev1) / 1e3, 1e-4)
-    reps = args.reps if args.reps > 0 else int(min(200, max(5, np.ceil(0.4 / est))))
-    if world > 1:
-        r = torch.tensor([reps], device=dev)
-        dist.all_reduce(r, op=dist.ReduceOp.MAX)
-        reps = int(r.item())
+    align()
+    runner.train_steps(K)
+    align()
     sampler = ClockSampler(local_rank)
     sampler.start()
     if args.profile_range:                      # ncu --profile-from-start off: capture only the steady-state steps
         torch.cuda.cudart().cudaProfilerStart()
-    blocks = timed_blocks(lambda: runner.train_steps(K), reps, world, dev)
+    blocks = timed_blocks(lambda: runner.train_steps(K), 1, world, dev)
     if args.profile_range:
         torch.cuda.cudart().cudaProfilerStop()
     clocks = sampler.summary()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(runner, args.dump_outputs)
     t_med = float(np.median(blocks))
     value = whole_job_value(N * K, blocks, world)           # every rank processes N*K rays per block (weak scaling)
 
@@ -398,19 +397,18 @@ def measure_config(args, c, name, rank, world, local_rank, dev, with_kernel=True
 
     for _ in range(5):
         step_e2e()
-    e2e_reps = max(3, min(reps, 25))
-    e2e_blocks = timed_blocks(e2e_block, e2e_reps, world, dev)
+    e2e_blocks = timed_blocks(e2e_block, 1, world, dev)
     t_e2e = float(np.median(e2e_blocks))
     e2e_value = world * N * K / t_e2e
 
     res = {'value': value, 'ms_per_step': 1e3 * t_med / K, 'steps_per_s': K / t_med, 'clocks': clocks,
-           'timing': {'reps': reps, 'block_steps': K, 'block_ms_median': 1e3 * t_med, 'block_ms_min': 1e3 * min(blocks), 'block_ms_max': 1e3 * max(blocks),
-                      'rule': 'median over reps of the max-over-ranks CUDA-event time of one K-step block (barrier + synchronize on both sides of every block)'},
-           'e2e': {'value': e2e_value, 'unit': 'rays/s', 'h2d_bytes_per_step': N * 12 * 4, 'd2h_bytes_per_step': 32, 'steps': K, 'reps': e2e_reps,
-                   'ms_per_step': 1e3 * t_e2e / K, 'block_ms_min': 1e3 * min(e2e_blocks), 'block_ms_max': 1e3 * max(e2e_blocks)},
+           'timing': {'timed_steps': K, 'block_ms': 1e3 * t_med,
+                      'rule': 'max-over-ranks CUDA-event time of the K timed steps (barrier + synchronize on both sides)'},
+           'e2e': {'value': e2e_value, 'unit': 'rays/s', 'h2d_bytes_per_step': N * 12 * 4, 'd2h_bytes_per_step': 32, 'steps': K,
+                   'ms_per_step': 1e3 * t_e2e / K},
            'ray_pool': int(runner.rays.shape[0]), 'setup_s': round(t_setup, 1), 'n_params': n_params}
     launches_per_step = (7 if DEFER_TABLE else 6) + (1 if c.get('eik', 0) > 0 else 0)   # prologue, ray march, operand pack, fused step, pose backward, Adam (1 | 2: small segments + table, bookkeeping on the last block of either) [+ eikonal count pass]
-    res['gpu_launches'] = launches_per_step * K * reps
+    res['gpu_launches'] = launches_per_step * K
     if not with_kernel:
         return res
 
@@ -453,12 +451,30 @@ def measure_config(args, c, name, rank, world, local_rank, dev, with_kernel=True
     return res
 
 
+DUMP_TABLE_ROWS = 1 << 18     # hash-table rows in the dump (all of them when the table is smaller)
+
+
+def dump_outputs(runner, out_dir):
+    """What a caller of train_steps has after its last step, as float32 .npy files (2 MB + the MLP and per-frame parameters)."""
+    runner.synchronize_parameters()                         # the last step's deferred table update
+    torch.cuda.synchronize()
+    os.makedirs(out_dir, exist_ok=True)
+    table = runner.table
+    rows = np.sort(np.random.default_rng(0).choice(table.shape[0], size=min(table.shape[0], DUMP_TABLE_ROWS), replace=False))
+    out = {'losses': runner._step_buf['losses'], 'mlp_params': runner.mlp_flat,
+           'hash_table_sample': table[torch.from_numpy(rows).to(table.device)]}
+    for key, name in (('pose_array', 'pose_params'), ('feature_array', 'frame_features')):
+        if runner.models[key] is not None:
+            out[name] = runner.models[key].data.data
+    for name, t in out.items():
+        np.save(os.path.join(out_dir, name + '.npy'), t.detach().float().cpu().numpy())
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=20)
+    ap.add_argument('--steps', type=int, default=20, help='timed steps of each measurement (value, e2e)')
     ap.add_argument('--warmup', type=int, default=20)
-    ap.add_argument('--reps', type=int, default=0, help='timed repetitions of the K-step block (0: enough for >= ~0.4 s, 5..200)')
     ap.add_argument('--impl', default='ours', choices=['ours', 'reference'])
     ap.add_argument('--config', default='C2', choices=list(CONFIGS))
     ap.add_argument('--cpu-rays', type=int, default=0, help='rays per step of the CPU baseline (0: the full batch unless a step would exceed ~20 s)')
@@ -466,7 +482,12 @@ def main():
     ap.add_argument('--no-config4', action='store_true', help='N > 1 only: skip the extra BASELINE configs[3] measurement (C3 x N)')
     ap.add_argument('--profile-range', action='store_true', help='bracket the timed steps with cudaProfilerStart/Stop (for ncu)')
     ap.add_argument('--eager', action='store_true', help='disable CUDA-graph replay of the step (launch the kernels one by one)')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write what the last timed step computed to DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be >= 1')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs dumps the timed path of --impl ours')
     c = CONFIGS[args.config]
     rank = int(os.environ.get('RANK', 0))
     world = int(os.environ.get('WORLD_SIZE', 1))

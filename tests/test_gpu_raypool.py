@@ -1,11 +1,10 @@
-"""GPU: the device-side ray-pool construction (SURVEY 8(f)-3) against the REFERENCE's own functions, imported from its Python under the
-stub modules of tests/golden/ref_shims.py (oracle/_ref/py on the GPU box, /root/reference in the build container):
-  NerfRunner.make_frame_rays (nerf_runner.py:246-316) incl. compute_near_far_and_filter_rays (:39-65) and the cv2 mask dilation,
+"""GPU: the device-side ray-pool construction (SURVEY 8(f)-3) against the REFERENCE's own functions:
+  NerfRunner.make_frame_rays (nerf_runner.py:246-316) incl. compute_near_far_and_filter_rays (:39-65) and the cv2 mask dilation, through
+  golden rows made by the reference's Python (tests/golden/make_golden_runner.py -> ref_gpu_frame_rays.npz),
   and the octree-cloud denoise of __init__ (:178-195, inline there: restated with the same scipy cKDTree call).
 The occupancy trace inside make_frame_rays goes through the product's OctreeManager in both (kaolin is absent)."""
 import os
 import sys
-import types
 
 import numpy as np
 import pytest
@@ -13,38 +12,27 @@ import torch
 
 pytestmark = pytest.mark.gpu
 HERE = os.path.dirname(os.path.abspath(__file__))
-REPO = os.path.dirname(HERE)
-
-
-def _reference():
-    sys.path.insert(0, os.path.join(HERE, 'golden'))
-    import ref_shims
-    ref_py = '/root/reference' if os.path.isdir('/root/reference') else os.path.join(REPO, 'oracle', '_ref', 'py')
-    if not os.path.exists(os.path.join(ref_py, 'nerf_runner.py')):
-        pytest.skip('reference Python not staged (oracle/build_ref.py stage_py)')
-    return ref_shims.import_reference(ref_py)
+sys.path.insert(0, os.path.join(HERE, 'golden'))
 
 
 def _runner(denoise):
-    from bundlesdf_b200 import synthetic as syn
-    from bundlesdf_b200.nerf_runner import NerfRunner
-    seq = syn.make_sequence(4, H=120, W=160, device='cuda', seed=5, pose_noise=True)
-    cfg = syn.default_cfg(N_rand=128, N_samples=32, N_samples_around_depth=32, num_levels=4, finest_res=128, log2_hashmap_size=12,
-                          sc_factor=seq['sc_factor'], translation=seq['translation'].tolist(), denoise_depth_use_octree_cloud=denoise)
-    r = NerfRunner(cfg, seq['images'], seq['depths'], seq['masks'], None, seq['poses'], seq['K'], build_octree_pcd=syn.PointCloud(seq['pcd_normalized']))
-    return r, seq
+    import make_golden_runner as M
+    return M.frame_rays_runner(denoise)
 
 
-def test_make_frame_rays_matches_the_reference():
-    nh, nr, U = _reference()
+def test_make_frame_rays_matches_the_reference(golden_dir):
+    import make_golden_runner as M
+    g = np.load(os.path.join(golden_dir, 'ref_gpu_frame_rays.npz'))
     ours, seq = _runner(False)
-    fake = types.SimpleNamespace(masks=ours.masks, images=ours.images, depths=ours.depths, poses=np.asarray(ours.poses), K=ours.K, H=ours.H, W=ours.W,
-                                 cfg=ours.cfg, occ_masks=None, normal_maps=None, octree_m=ours.octree_m)
-    for fid in (0, 2):
-        want = nr.NerfRunner.make_frame_rays(fake, fid)                        # numpy float64 [R, 12]
-        got = ours.make_frame_rays(fid).cpu().numpy()
-        assert got.shape == want.shape and got.shape[0] > 500, (got.shape, want.shape)
-        np.testing.assert_allclose(got, want, rtol=2e-5, atol=2e-5)            # fp32 on the device vs fp64 numpy; same rows in the same order
+    for fid in M.FRAME_RAYS_FRAMES:
+        got = ours.make_frame_rays(fid).cpu().numpy().astype(np.float64)
+        n = int(g[f'n_rows_{fid}'])
+        assert got.shape == (n, 12) and n > 500, (got.shape, n)
+        # fp32 on the device vs fp64 numpy; same rows in the same order: a seeded sample row by row, every row through the column sums
+        np.testing.assert_allclose(got[M.frame_rays_sample(n)], g[f'rows_{fid}'], rtol=2e-5, atol=2e-5)
+        tol = 2e-5 * (n + g[f'col_abs_sum_{fid}'])
+        for have, want in ((got.sum(0), g[f'col_sum_{fid}']), (np.abs(got).sum(0), g[f'col_abs_sum_{fid}'])):
+            assert (np.abs(have - want) <= tol).all(), (fid, have, want)
 
 
 def test_octree_cloud_denoise_matches_ckdtree():

@@ -1,61 +1,33 @@
 """GPU: a whole training run (the reference's n_step = 500) of the drop-in NerfRunner against the reference's OWN NerfRunner.train_loop
 (nerf_runner.py:679-852, run verbatim on top of its own CUDA extensions, oracle/ref_train_loop.py) on the same data from the same initial
-parameters. The two draw different sample noise (torch.rand there, in-kernel Philox here), so the runs are compared as what they are —
-two realisations of the same stochastic optimisation: the loss level they reach, the SDF field and the surface normals they learn.
+parameters, as recorded by tests/golden/make_golden_runner.py (ref_gpu_training_500.npz). The two draw different sample noise
+(torch.rand there, in-kernel Philox here), so the runs are compared as what they are — two realisations of the same stochastic
+optimisation: the loss level they reach, the SDF field and the surface normals they learn.
 
 Tolerances (stated, not tuned per run): final loss within 20 %; SDF fields correlate > 0.9 and agree in sign on > 90 % of the probes inside
 the truncation band; normals of the two fields within the band have a mean cosine > 0.8."""
+import os
+import sys
+
 import numpy as np
 import pytest
 import torch
 
 pytestmark = pytest.mark.gpu
+sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden'))
 
 
-def _probe_points(r, step=0.04):
-    """Lattice points of the normalised cube that fall into occupied cells (what extract_mesh sweeps, nerf_runner.py:1351-1380)."""
-    ax = np.arange(-1 + 0.5 * step, 1, step, dtype=np.float32)
-    g = torch.tensor(np.stack(np.meshgrid(ax, ax, ax, indexing='ij'), -1).reshape(-1, 3)).cuda()
-    return g[r.octree_m.get_center_ids(g) >= 0]
-
-
-def test_500_steps_track_the_references_own_training():
-    from oracle import ref_train_loop as RT
-    try:
-        RT.reference_modules()
-    except RuntimeError as e:
-        pytest.skip(str(e))
-    from bundlesdf_b200 import synthetic as syn
-    from bundlesdf_b200.nerf_runner import NerfRunner, set_seed
+def test_500_steps_track_the_references_own_training(golden_dir):
+    import make_golden_runner as M
+    from bundlesdf_b200.nerf_runner import set_seed
+    gold = np.load(os.path.join(golden_dir, 'ref_gpu_training_500.npz'))
     n_step = 500
-    set_seed(0)
-    seq = syn.make_sequence(6, H=120, W=160, device='cuda', seed=3, pose_noise=True)
-    cfg = syn.default_cfg(N_rand=512, N_samples=64, N_samples_around_depth=64, num_levels=16, finest_res=256, log2_hashmap_size=14, amp=True,
-                          sc_factor=seq['sc_factor'], translation=seq['translation'].tolist(), n_step=n_step, defer_table_update=True)
-    r = NerfRunner(cfg, seq['images'], seq['depths'], seq['masks'], None, seq['poses'], seq['K'], build_octree_pcd=syn.PointCloud(seq['pcd_normalized']))
-    ref = RT.build_reference_runner(r)                    # the reference's own create_nerf / create_optimizer / GradScaler(65536)
-    with torch.no_grad():                                 # same starting point: the reference's initialisation
-        r.models['embed_fn'].embeddings.copy_(ref.models['embed_fn'].embeddings)
-        if r.table_f16 is not None:
-            r.table_f16.copy_(r.table)
-        r.models['model'].load_state_dict(ref.models['model'].state_dict())
-
-    # ---- the reference: 500 x train_loop, loss captured at the GradScaler like tests/golden/make_golden_step.py does
-    ref_losses = []
-    real_scale = ref.amp_scaler.scale
-
-    def scale(loss):
-        ref_losses.append(loss.detach().float())
-        return real_scale(loss)
-    ref.amp_scaler.scale = scale
-    set_seed(1)
-    ref.data_loader = RT.reference_modules()[1].DataLoader(rays=ref.rays, batch_size=cfg['N_rand'])
-    for _ in range(n_step):
-        batch = next(ref.data_loader)
-        ref.data_loader.batch_ray_ids = ref.data_loader.batch_ray_ids.to(batch.device)      # torch >= 2 indexing rule, see oracle/ref_train_loop.py
-        ref.train_loop(batch)
-        ref.global_step += 1
-    ref_losses = torch.stack(ref_losses).cpu().numpy()
+    r = M.training_runner(n_step)
+    cfg = r.cfg
+    # the reference's run (tests/golden/make_golden_runner.py) started from this runner's initial parameters: 500 x train_loop, the loss of
+    # every step captured at the GradScaler
+    ref_losses = gold['losses']
+    assert ref_losses.shape == (n_step,)
 
     # ---- ours: the same number of steps through train_steps (10-step graph blocks), loss read after every block
     set_seed(1)
@@ -81,17 +53,17 @@ def test_500_steps_track_the_references_own_training():
     assert last_r < 0.5 * ref_losses[0] and last_o < 0.5 * ref_losses[0]
     assert abs(last_o - last_r) <= 0.2 * last_r, (last_o, last_r)
 
-    # ---- the fields
-    pts = _probe_points(r)
+    # ---- the fields, at the probe points the reference's field was evaluated at (a seeded sample of M.probe_points)
+    pts = torch.from_numpy(gold['probe_points']).cuda()
     so = r.run_network_density(pts, get_normals=True)[0]
-    sr = ref.run_network_density(pts.clone(), get_normals=True)[0].detach()
-    sdf_o, sdf_r = so[:, 0].cpu().numpy(), sr[:, 0].cpu().numpy()
+    sr = gold['sdf_normals']
+    sdf_o, sdf_r = so[:, 0].cpu().numpy(), sr[:, 0]
     band = (np.abs(sdf_r) < 0.9) | (np.abs(sdf_o) < 0.9)
     assert band.sum() > 200, band.sum()
     corr = np.corrcoef(sdf_o[band], sdf_r[band])[0, 1]
     sign = (np.sign(sdf_o[band]) == np.sign(sdf_r[band])).mean()
     near = (np.abs(sdf_r) < 0.5) & (np.abs(sdf_o) < 0.5)
-    no, nr = so[:, 1:].cpu().numpy()[near], sr[:, 1:].cpu().numpy()[near]
+    no, nr = so[:, 1:].cpu().numpy()[near], sr[:, 1:][near]
     cos = (no * nr).sum(-1) / np.maximum(np.linalg.norm(no, axis=-1) * np.linalg.norm(nr, axis=-1), 1e-12)
     print(f'probes {len(pts)}, in band {band.sum()}: sdf correlation {corr:.4f}, sign agreement {sign:.4f}; normals on {near.sum()} probes: mean cosine {cos.mean():.4f}')
     assert corr > 0.9 and sign > 0.9, (corr, sign)

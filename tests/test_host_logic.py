@@ -158,21 +158,25 @@ def test_ray_walk_as_merge_of_axis_crossings_is_bit_identical():
         assert (a[:, 0, 0] != 0).sum() > N // 2
 
 
-def test_reference_shims_reimport_once_the_extensions_are_there():
-    """tests/golden/ref_shims.import_reference: the CPU-side golden tests import the reference WITHOUT its CUDA extensions (its
-    `from mycuda import common` then fails silently); a later import WITH them (oracle/ref_train_loop.py on the GPU box) has to
-    produce fresh modules that see the extensions, or the reference's train_loop dies on `common` mid-suite."""
-    import importlib.util
+def test_reference_shims_reimport_once_the_extensions_are_there(tmp_path):
+    """tests/golden/ref_shims.import_reference: the CPU-side golden generators import the reference WITHOUT its CUDA extensions (its
+    `from mycuda import common` then fails silently); a later import WITH them (oracle/ref_train_loop.py on a GPU) has to
+    produce fresh modules that see the extensions, or the reference's train_loop dies on `common`. The modules here are stand-ins with
+    the reference's import chain (Utils.py:28-31 imports `common` under try/except; nerf_helpers and nerf_runner star-import Utils)."""
     import sys
     import types
-    ref_dir = '/root/reference' if os.path.isdir('/root/reference') else os.path.join(REPO, 'oracle', '_ref', 'py')
-    if not os.path.exists(os.path.join(ref_dir, 'nerf_runner.py')):
-        pytest.skip('reference sources not present')
+    (tmp_path / 'Utils.py').write_text('try:\n    from mycuda import common\nexcept Exception:\n    pass\n')
+    (tmp_path / 'nerf_helpers.py').write_text('from Utils import *\n')
+    (tmp_path / 'nerf_runner.py').write_text('from nerf_helpers import *\nfrom Utils import *\n')
+    ref_dir = str(tmp_path)
     sys.path.insert(0, os.path.join(REPO, 'tests', 'golden'))
     import ref_shims
     saved = {k: sys.modules.get(k) for k in ('Utils', 'nerf_helpers', 'nerf_runner', 'mycuda', 'mycuda.common', 'gridencoder')}
+    for k in ('Utils', 'nerf_helpers', 'nerf_runner'):
+        sys.modules.pop(k, None)
     try:
         _, nr_plain, _ = ref_shims.import_reference(ref_dir)
+        assert not hasattr(nr_plain, 'common')
         fake_c, fake_g = types.ModuleType('common_fake'), types.ModuleType('gridencoder_fake')
         _, nr_ext, _ = ref_shims.import_reference(ref_dir, mycuda_common=fake_c, mycuda_gridencoder=fake_g)
         assert nr_ext is not nr_plain and nr_ext.common is fake_c
@@ -182,6 +186,7 @@ def test_reference_shims_reimport_once_the_extensions_are_there():
                 sys.modules.pop(k, None)
             else:
                 sys.modules[k] = v
+        sys.path.remove(ref_dir)
 
 
 def test_device_cursor_protocol_walks_the_same_batches_as_the_per_step_loader():
@@ -218,23 +223,18 @@ def test_device_cursor_protocol_walks_the_same_batches_as_the_per_step_loader():
 
 
 @pytest.mark.parametrize('decay', ['', 'linear', 'exp'])
-def test_truncation_schedule_matches_the_references_own_method(decay):
+def test_truncation_schedule_matches_the_references_own_method(golden_dir, decay):
     """get_truncation (nerf_runner.py:663-676): the product's host formula (which also fills the device table of the annealed schedule) and the
     oracle's, against the reference's own NerfRunner.get_truncation called on a stand-in self — every step of a 500-step run, bit for bit."""
-    import sys
     import types
-    ref_dir = '/root/reference' if os.path.isdir('/root/reference') else os.path.join(REPO, 'oracle', '_ref', 'py')
-    if not os.path.exists(os.path.join(ref_dir, 'nerf_runner.py')):
-        pytest.skip('reference sources not present')
-    sys.path.insert(0, os.path.join(REPO, 'tests', 'golden'))
-    import ref_shims
     from bundlesdf_b200.nerf_runner import NerfRunner
     from oracle import nof_oracle as O
-    _, nr, _ = ref_shims.import_reference(ref_dir)
+    gold = np.load(os.path.join(golden_dir, 'ref_py_truncation.npz'))   # tests/golden/make_golden_runner.py
     cfg = dict(trunc_decay_type=decay, trunc_start=0.03, trunc=0.01, n_step=500, sc_factor=3.7)
-    for g in list(range(0, 40)) + [123, 124, 125, 126, 250, 499, 500, 501]:
+    steps, wants = gold['steps'], gold['trunc_' + (decay or 'const')]
+    assert list(steps) == list(range(0, 40)) + [123, 124, 125, 126, 250, 499, 500, 501]
+    for g, want in zip(steps.tolist(), wants.tolist()):
         me = types.SimpleNamespace(cfg=cfg, global_step=g)
-        want = nr.NerfRunner.get_truncation(me)
         assert NerfRunner.get_truncation(me) == want
         assert NerfRunner.get_truncation(me, step=g) == want
         assert O.get_truncation(cfg, g) == want
