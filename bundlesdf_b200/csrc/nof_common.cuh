@@ -89,7 +89,7 @@ __device__ __forceinline__ void red_add(float* addr, float a) {
 }
 
 // Philox4x32-10 counter RNG -> uniform [0,1) floats (same construction torch / curand use; the stream itself is
-// ours — parity tests inject t_rand instead).
+// ours: tests/test_gpu_ray_march.py pins the ray march's draws to a numpy restatement checked on the Random123 vectors).
 __device__ __forceinline__ uint4 philox4x32_10(uint4 ctr, uint2 key) {
   const uint32_t M0 = 0xD2511F53u, M1 = 0xCD9E8D57u, W0 = 0x9E3779B9u, W1 = 0xBB67AE85u;
 #pragma unroll

@@ -557,6 +557,45 @@ def stratified_np(S, near, far, t_rand):
     return z.astype(f32)
 
 
+PHILOX_M = (0xD2511F53, 0xCD9E8D57)      # round multipliers of Philox4x32
+PHILOX_W = (0x9E3779B9, 0xBB67AE85)      # key schedule increments (golden ratio, sqrt(3) - 1)
+
+
+def philox4x32_10(ctr, key):
+    """Philox4x32-10 (Salmon, Moraes, Dror, Shaw, "Parallel random numbers: as easy as 1, 2, 3", SC'11; the Random123 library's
+    philox4x32_10), from its definition: ten rounds; round i uses key_i = key_0 + i * W (mod 2^32 per word) and maps
+    (c0, c1, c2, c3) -> (hi(M1 c2) ^ c1 ^ k0, lo(M1 c2), hi(M0 c0) ^ c3 ^ k1, lo(M0 c0)) with hi/lo the halves of the 64-bit product.
+    ctr: uint32 array [..., 4]; key: uint32 array [..., 2] (broadcast against ctr). Returns uint32 [..., 4]."""
+    mask = np.uint64(0xFFFFFFFF)
+    ctr = np.asarray(ctr, np.uint64)
+    key = np.asarray(key, np.uint64)
+    c0, c1, c2, c3 = (ctr[..., i] for i in range(4))
+    m0, m1 = np.uint64(PHILOX_M[0]), np.uint64(PHILOX_M[1])
+    for i in range(10):
+        k0 = (key[..., 0] + np.uint64(i * PHILOX_W[0])) & mask
+        k1 = (key[..., 1] + np.uint64(i * PHILOX_W[1])) & mask
+        p0, p1 = m0 * c0, m1 * c2                  # 32 x 32 -> 64 bits: exact in uint64
+        c0, c1, c2, c3 = (p1 >> np.uint64(32)) ^ c1 ^ k0, p1 & mask, (p0 >> np.uint64(32)) ^ c3 ^ k1, p0 & mask
+    return np.stack(np.broadcast_arrays(c0, c1, c2, c3), -1).astype(np.uint32)
+
+
+def march_uniforms(N, S, seed, offset):
+    """The [N, S] float32 jitter the ray march draws when no t_rand is given (the stream is the project's own, see
+    nof_ray_march in include/nof.h): element [r, s] is word s & 3 of philox4x32_10(ctr=(r, s >> 2, offset mod 2^32, offset >> 32),
+    key=(seed mod 2^32, seed >> 32)), mapped to [0, 1) by (x >> 8) * 2^-24. The words past S in the last group are unused.
+    `offset` is the launch offset plus the device tick (NofMarchCfg.offset + *offset_ptr), 64-bit."""
+    seed, offset = int(seed) & (2 ** 64 - 1), int(offset) & (2 ** 64 - 1)
+    G = (S + 3) // 4
+    ctr = np.zeros((N, G, 4), np.uint32)
+    ctr[..., 0] = np.arange(N, dtype=np.uint32)[:, None]
+    ctr[..., 1] = np.arange(G, dtype=np.uint32)[None, :]
+    ctr[..., 2] = offset & 0xFFFFFFFF
+    ctr[..., 3] = offset >> 32
+    key = np.array([seed & 0xFFFFFFFF, seed >> 32], np.uint32)
+    words = philox4x32_10(ctr, key).reshape(N, 4 * G)[:, :S]
+    return ((words >> np.uint32(8)).astype(np.float32) * np.float32(2.0 ** -24)).astype(np.float32)
+
+
 def rays_world_np(batch, tf12):
     """Unit camera dir, world origin, world unit dir per ray (nerf_runner.py:1045-1057) in the exact fp32 operation
     order of the CUDA sampler: nrm=sqrt((dx*dx+dy*dy)+dz*dz); u=d/nrm; dw_i=(R_i0*u0+R_i1*u1)+R_i2*u2.
